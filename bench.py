@@ -2,6 +2,7 @@
 """bench.py -- frames/sec of MEGA R-101 inference (1000x600) on B200, with parity, roofline and CPU baseline.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--arch mega_r101|rdn_r101|fgfa_r101]
+                    [--dump-outputs DIR]
 
 A "step" of the default workload (configs[1] of BASELINE.json) is one pass of the MEGA R-101 hot path at 600x1000 in
 steady state: the new look-ahead local frame and the new global frame of every key frame of the step go through
@@ -23,6 +24,11 @@ THAT MEETS THE BAR (`config.precision`); every measured mode is listed under `mo
 Output: ONE JSON line (driver contract): `value` = key frames/s with inputs resident in HBM (CUDA events, max over ranks),
 `e2e` = the same through the public model API with pinned-host inputs and a host read of the detections, `roofline` for
 the tensor-core kernels, `cpu_baseline` = the reference path on this box's host cores on a bounded sample.
+
+--dump-outputs DIR: after the timed steps, the detections the last device-resident step returned (what a caller of
+that step receives) go to DIR as float32 .npy files, one set per timed mode and key frame of the step:
+<precision>_frame<g>_{boxes,scores,labels}.npy. Inputs and weights are seeded, so the same arguments give the same
+inputs on every run and two builds can be compared output for output.
 
 N > 1 (torchrun): ONE video stream, frame-parallel (SURVEY.md section 8e): per step every rank runs the per-frame branch
 of its own (local, global) frame pair, NCCL all-gathers exchange the fixed-size ROI-feature payloads (and, in the
@@ -100,7 +106,29 @@ def parse():
     ap.add_argument("--cpu-sample-frames", type=int, default=3)
     ap.add_argument("--skip-cpu-baseline", action="store_true")
     ap.add_argument("--skip-roofline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the detections of the last timed step to DIR/<name>.npy (float32)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
+
+
+def detection_arrays(prefix, dets):
+    """{name: float32 array} of one step's detections (a Detections or a list of them, one per key frame)"""
+    import numpy as np
+    out = {}
+    for g, det in enumerate(dets if isinstance(dets, list) else [dets]):
+        for field, t in zip(("boxes", "scores", "labels"), det.to_host()):
+            out["%s_frame%d_%s" % (prefix, g, field)] = t.numpy().astype(np.float32)
+    return out
+
+
+def dump_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in sorted(arrays.items()):
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 DEFAULT_PIPELINE = 0   # --pipeline 1 (N = 1, strict mode): the aggregation of a batch overlaps the per-frame branch of the next one
@@ -369,12 +397,14 @@ class MegaBench:
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
             for i in range(args.steps):
-                step_dev(i)
+                last = step_dev(i)
             e1.record()
             self.barrier()
             if self.sampler is not None:
                 self.sampler.mark()
             dev_ms = e0.elapsed_time(e1)
+            if args.dump_outputs:          # read before the next step overwrites the engine's static detection buffers
+                res["outputs"] = detection_arrays(precision, last)
             # ---- timed region B: end to end: pinned host inputs -> detections on the host (the public model API at N=1)
             for i in range(max(args.warmup, 3)):
                 step_e2e()
@@ -492,15 +522,6 @@ def roofline_pass(eng, step, reps=3):
     ms = sum(r[0].elapsed_time(r[1]) for r in rec) / reps
     fl = sum(r[2] for r in rec) / reps
     n = max(len(rec) // reps, 1)
-    try:        # per-launch table of the last eager step (diagnostics; gpurun_out/ is scratch)
-        rows = [dict(r[3], us=round(r[0].elapsed_time(r[1]) * 1e3, 2), gflop=round(r[2] / 1e9, 3)) for r in rec[-n:]]
-        for r in rows:
-            r.pop("layers", None)
-        os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-        with open(os.path.join(ROOT, "gpurun_out", "launch_times.json"), "w") as fh:
-            json.dump(rows, fh)
-    except Exception:
-        pass
     # the dominant launch = the one with the largest share of the step's tensor-core time
     dom, best = None, -1.0
     for i in range(n):
@@ -589,17 +610,10 @@ def run_mega(args, rank, world):
                 roofs[p] = roofline_pass(e, lambda i, e=e, md=md, nb=nb: e.stepn_batched(md[i % nb], mb.w, mb.h))
             else:
                 roofs[p] = roofline_pass(e, lambda i, e=e: e.step_batched(mb.pairs_dev[i % 16], mb.w, mb.h))
-            if p == head:
-                try:
-                    os.replace(os.path.join(ROOT, "gpurun_out", "launch_times.json"),
-                               os.path.join(ROOT, "gpurun_out", "launch_times_%s.json" % p))
-                except OSError:
-                    pass
     if rank != 0:
         return None
-    from mega_core.b200 import ops
-    os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
-    ops.save_tuned(os.path.join(ROOT, "gpurun_out", "tuned_b200.json"))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: v for p in modes for k, v in results[p]["outputs"].items()})
     kf_step_roof = fps                      # the roofline pass runs the single-GPU step
     line = {
         "metric": METRIC, "value": R["value"], "unit": "frames/s", "n_gpus": world, "steps": args.steps,
@@ -694,10 +708,12 @@ def run_windowed(args, rank, world):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for i in range(args.steps):
-            eng.step(pdev[i % 16], w, h)
+            last = eng.step(pdev[i % 16], w, h)
         e1.record()
         torch.cuda.synchronize(dev)
         dev_ms = e0.elapsed_time(e1)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, detection_arrays(precision, last))
         for i in range(3):
             model(infos(t))[0].to("cpu")
             t += 1

@@ -7,6 +7,7 @@ what the GPU-side tests and the CPU oracle tests compare against on a box withou
 reference.
 """
 import importlib.util
+import json
 import os
 import sys
 import types
@@ -460,6 +461,27 @@ def golden_base(h=192, w=320):
             "scores": res.get_field("scores").clone(), "labels": res.get_field("labels").clone()}
 
 
+# ------------------------------------------------------------------ 4. the YAML configs tools/test_net.py is run with
+CONFIGS = ("configs/BASE_RCNN_1gpu.yaml", "configs/MEGA/vid_R_101_C4_MEGA_1x.yaml", "configs/RDN/vid_R_101_C4_RDN_1x.yaml",
+           "configs/FGFA/vid_R_101_C4_FGFA_1x.yaml", "configs/DFF/vid_R_101_C4_DFF_1x.yaml", "configs/vid_R_50_C4_1x.yaml")
+
+
+def golden_configs():
+    """the settings of each config, by path, as yaml.safe_load reads them (what cfg.merge_from_file merges)"""
+    import yaml
+    out = {}
+    for rel in CONFIGS:
+        with open(os.path.join(ref_import.REFERENCE, rel)) as fh:
+            out[rel] = yaml.safe_load(fh)
+    return out
+
+
+def write_golden_configs():
+    with open(os.path.join(GOLD, "reference_configs.json"), "w") as fh:
+        json.dump(golden_configs(), fh, indent=1, sort_keys=True)
+        fh.write("\n")
+
+
 def main():
     os.makedirs(GOLD, exist_ok=True)
     torch.set_num_threads(8)
@@ -473,6 +495,9 @@ def main():
     if "dff" in only:
         torch.save(golden_dff(), os.path.join(GOLD, "dff_r101_192x320.pt"))
         return
+    if "configs" in only:
+        write_golden_configs()
+        return
     print("[1] reference unit-test vectors")
     torch.save(golden_from_reference_tests(), os.path.join(GOLD, "reference_unit_vectors.pt"))
     print("[2] op-level reference outputs")
@@ -483,6 +508,8 @@ def main():
     torch.save(golden_rdn(), os.path.join(GOLD, "rdn_r101_192x320.pt"))
     torch.save(golden_fgfa(), os.path.join(GOLD, "fgfa_r101_192x320.pt"))
     torch.save(golden_dff(), os.path.join(GOLD, "dff_r101_192x320.pt"))
+    print("[4] configs")
+    write_golden_configs()
     for f in sorted(os.listdir(GOLD)):
         print("  wrote", f, os.path.getsize(os.path.join(GOLD, f)), "bytes")
 

@@ -1,10 +1,14 @@
 """Runs the UNMODIFIED reference dataset classes (mega_core/data/datasets/vid*.py) with the reference's CPU transforms on
-a (synthetic) ImageNet-VID tree and dumps every test item -- the checker of mega_core.data.datasets in
-tests/test_datasets_cpu.py. TEST INFRASTRUCTURE; separate process (it imports the reference's `mega_core`).
-Usage: python oracle/run_ref_datasets.py <data_dir> <out.pt>"""
+the synthetic ImageNet-VID tree of tests/test_datasets_cpu.make_tree and writes every test item as the fixture the
+checker of mega_core.data.datasets in tests/test_datasets_cpu.py compares with: image tensors as fingerprints (dtype,
+shape, SHA-256 of the bytes), paths relative to the tree. TEST INFRASTRUCTURE; separate process (it imports the
+reference's `mega_core`).
+Usage (needs the reference checkout, see ref_import.py):
+    python oracle/run_ref_datasets.py tests/golden/reference_datasets.pt"""
 import importlib.util
 import os
 import sys
+import tempfile
 import types
 
 import numpy as np
@@ -12,7 +16,9 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.join(os.path.dirname(HERE), "tests"))
 import ref_import  # noqa: E402
+from test_datasets_cpu import fingerprint, make_tree  # noqa: E402
 
 
 def load(name, path):
@@ -23,7 +29,14 @@ def load(name, path):
     return mod
 
 
-def main(data_dir, out_path):
+def main(out_path):
+    with tempfile.TemporaryDirectory() as data_dir:
+        make_tree(data_dir)
+        out = run(data_dir)
+    torch.save(out, out_path)
+
+
+def run(data_dir):
     ref_import.setup()
     ref = os.path.join(ref_import.REFERENCE, "mega_core")
     # the dataset files, by path: the package __init__ chain pulls in COCO / Cityscapes helpers that are not installed
@@ -58,15 +71,13 @@ def main(data_dir, out_path):
         items = []
         for i in range(len(ds)):
             images, target, idx = ds[i]
-            if isinstance(images, dict):
-                images = {k: v for k, v in images.items() if k != "transforms"}
-            items.append({"images": images, "boxes": target.bbox.clone(), "labels": target.get_field("labels").clone(),
-                          "size": target.size, "idx": idx})
+            items.append({"images": fingerprint(images, data_dir), "boxes": target.bbox.clone(),
+                          "labels": target.get_field("labels").clone(), "size": target.size, "idx": idx})
         out[key] = {"items": items, "img_info": [ds.get_img_info(i) for i in range(len(ds))],
                     "start_index": getattr(ds, "start_index", None)}
         os.remove(os.path.join(data_dir, "cache", "VID_val_videos_anno.pkl"))
-    torch.save(out, out_path)
+    return out
 
 
 if __name__ == "__main__":
-    main(sys.argv[1], sys.argv[2])
+    main(sys.argv[1])

@@ -4,6 +4,9 @@ import json
 import os
 import subprocess
 import sys
+import types
+
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -24,5 +27,27 @@ def test_reference_arm_prints_the_contract_line():
 
 def test_b200_arm_flags():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--wave", "--no-wave", "--precision"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--wave", "--no-wave", "--precision", "--dump-outputs"):
         assert flag in out.stdout
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True,
+                         text=True, timeout=120)
+    assert out.returncode != 0 and "--steps" in out.stderr
+
+
+def test_dump_outputs_writes_every_key_frame_as_float32(tmp_path):
+    """--dump-outputs: <precision>_frame<g>_{boxes,scores,labels}.npy for each key frame of the last step"""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+
+    def det(n):
+        return types.SimpleNamespace(to_host=lambda: (torch.rand(n, 4) * 100, torch.rand(n), torch.randint(1, 31, (n,))))
+
+    arrays = bench.detection_arrays("fp32x3", [det(3), det(0)])
+    bench.dump_outputs(str(tmp_path / "out"), arrays)
+    names = sorted(os.listdir(tmp_path / "out"))
+    assert names == sorted("fp32x3_frame%d_%s.npy" % (g, f) for g in range(2) for f in ("boxes", "scores", "labels"))
+    for name in names:
+        a = np.load(tmp_path / "out" / name)
+        assert a.dtype == np.float32 and np.array_equal(a, arrays[name[:-4]])
+    assert arrays["fp32x3_frame0_boxes"].shape == (3, 4) and arrays["fp32x3_frame1_labels"].shape == (0,)

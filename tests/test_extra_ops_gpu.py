@@ -84,7 +84,7 @@ def test_callable_submodules_match_the_oracle_pieces(cuda_dev):
     parts (generalized_rcnn_mega.py:145-158, :173-175, :208; rpn/rpn.py:213-243; extractors :657-676, :885-896) -- served
     by the detector's engine, against the oracle's functions of the same steps on the same inputs."""
     import mega_oracle as mo
-    from mega_core.b200 import synth
+    from mega_core.b200 import ops, synth
     from mega_core.modeling.detector import build_detection_model_from_state_dict
     from mega_core.structures.image_list import to_image_list
     sd = synth.make_state_dict("mega_r101_tiny", seed=3)
@@ -123,9 +123,14 @@ def test_callable_submodules_match_the_oracle_pieces(cuda_dev):
     # global pool: init + push lands in ring slot 0
     fe.init_memory()
     fe.init_global()
+    x_in = x.clone()
     fe.update_global(x)
     eng = model.engine
     assert eng.glob_pushed == 1 and eng.mem_pushed == 0
-    assert torch.allclose(eng.glob_x[:75].float(), x, atol=1e-6)
+    assert torch.equal(x, x_in)                                      # the caller's rows are left as they were
+    pushed = eng.glob_x[:75].float()
+    if ops.is_split16(eng.glob_x):                                   # strict mode stores the pool as split-fp16 pairs
+        pushed = ops.unpack_split16(pushed, torch.empty_like(pushed))
+    assert torch.allclose(pushed, x, atol=1e-6)
     with pytest.raises(NotImplementedError):
         fe((dfeats,), [key[0]], pre_calculate=False)

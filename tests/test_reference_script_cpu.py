@@ -1,10 +1,11 @@
-"""The reference's OWN evaluation script, unmodified -- /root/reference/tools/test_net.py -- executed against this
-package: its imports (`mega_core.config / data / engine.inference / modeling.detector / utils.*`) resolve here, the
-reference's YAML configs drive it, a synthetic ImageNet-VID tree in the reference layout stands in for the dataset, a
-checkpoint saved the way the reference's trainer saves it is loaded through DetectronCheckpointer, every frame goes
-through `model(images)` (MEGA R-101: window / global / memory state machine, look-ahead frames read from disk inside the
-model) and the VID evaluator writes result.txt. No GPU in this container, so the device ops run on the CPU stand-ins of
-tests/cpu_ops.py and the device check of the module is lifted (both test-only); on a B200 the same script runs as is."""
+"""The reference's OWN evaluation script, unmodified -- tools/test_net.py of the reference checkout the oracle
+imports (oracle/ref_import.py) -- executed against this package: its imports (`mega_core.config / data /
+engine.inference / modeling.detector / utils.*`) resolve here, the reference's YAML configs drive it, a synthetic
+ImageNet-VID tree in the reference layout stands in for the dataset, a checkpoint saved the way the reference's trainer
+saves it is loaded through DetectronCheckpointer, every frame goes through `model(images)` (MEGA R-101: window / global
+/ memory state machine, look-ahead frames read from disk inside the model) and the VID evaluator writes result.txt. The
+device ops run on the CPU stand-ins of tests/cpu_ops.py and the device check of the module is lifted (both test-only),
+so no GPU is needed; on a B200 the same script runs as is."""
 import os
 import runpy
 import sys
@@ -16,10 +17,12 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "tests"))
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(ROOT, "oracle"))
+from ref_import import REFERENCE as REF  # noqa: E402  (the checkout the oracle imports; MEGA_REFERENCE overrides it)
 
 
-@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "tools", "test_net.py")), reason="reference checkout not present")
+@pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "tools", "test_net.py")),
+                    reason="reference checkout not present (MEGA_REFERENCE names it)")
 def test_unmodified_tools_test_net_runs_on_this_package(tmp_path, monkeypatch):
     from cpu_ops import cpu_ops
     from test_datasets_cpu import CpuTransform, make_tree
