@@ -427,6 +427,45 @@ int mega_vid_match_host(const float* pred_boxes, int n_pred, const float* gt_box
                         int n_gt, float iou_thresh, double empty_weight, signed char* match_out,
                         double* pred_ignore_out);
 
+/* ---------------------------------------------------------------- device VID evaluator (added to ABI v6)
+ * These four symbols were added to v6 without changing anything before them, so mega_abi_version() stays 6.
+ * calc_detection_vid_prec_rec + calc_detection_vid_ap for up to 4 motion ranges in one pass
+ * (data/datasets/evaluation/vid/vid_eval.py:156-284, :287-343). Inputs are the BoxLists packed image after image:
+ *   detections: det_boxes [n_det,4] xyxy, det_scores [n_det], det_labels [n_det] int32 in [0, num_classes);
+ *   ground truth: gt_boxes [n_gt,4], gt_labels [n_gt], gt_motion [n_gt] fp64 motion IoU (NaN: none, never ignored;
+ *   gt_motion NULL: nothing is ignored); det_offsets / gt_offsets [n_img+1] int64 prefix sums of the per-image counts.
+ * Boxes satisfy x2 > x1 - 2 and y2 > y1 - 2. num_classes <= 512, n_ranges 1..4, n_det and n_gt < 2^31.
+ * ranges_host [n_ranges][2] = (lo, hi): a GT is ignored for a range when its motion IoU lies outside [lo, hi]
+ * (vid_eval.py:176-186); empty_weight_host [n_ranges]: the ignore weight of detections of a class without GT in the image
+ * (vid_eval.py:160-169, 206). Ranking rule: descending score, equal scores in the order of numpy's
+ * argsort(kind="stable")[::-1] inside each (image, class) and over each class (the reference's own argsort()[::-1] leaves
+ * equal scores in an unspecified order, vid_eval.py:191, :265). All four calls share one workspace of
+ * mega_vid_eval_workspace_bytes() bytes (-1: sizes out of range), run in stream order and are called in this order. */
+long long mega_vid_eval_workspace_bytes(long long n_det, long long n_gt, int num_classes, int n_ranges);
+/* Per (image, class): greedy matching for every range (vid_eval.py:188-250). match_out [n_ranges][n_det] int8 (1 =
+ * matched), ignore_out [n_ranges][n_det] fp64 (the reference's pred_ignore), n_pos_out [n_ranges][num_classes] int64
+ * (non-ignored GT, vid_eval.py:199), seen_out [num_classes] int32 (1 = label occurs in a prediction or GT: prec exists),
+ * det_count_out [num_classes] int32 detections per class. Zeroes its outputs itself. */
+int mega_vid_eval_match(const float* det_boxes, const float* det_scores, const int* det_labels,
+                        const long long* det_offsets, const float* gt_boxes, const int* gt_labels, const double* gt_motion,
+                        const long long* gt_offsets, int n_img, long long n_det, long long n_gt, int num_classes,
+                        int n_ranges, const double* ranges_host, const double* empty_weight_host, float iou_thresh,
+                        void* workspace, long long workspace_bytes, signed char* match_out, double* ignore_out,
+                        long long* n_pos_out, int* seen_out, int* det_count_out, void* stream);
+/* Stable radix sort of all detections by (class, score) ascending (vid_eval.py:260-268 for every class at once):
+ * order_out [n_det] = detection indices; class c occupies det_count[c] entries after those of the classes below it, and
+ * read backwards each class is in ranking order. */
+int mega_vid_eval_rank(long long n_det, long long n_gt, int num_classes, int n_ranges, void* workspace,
+                       long long workspace_bytes, int* order_out, void* stream);
+/* Per (class, range): tp / fp cumulative sums, prec = tp / (fp + tp + eps), rec = tp / n_pos (vid_eval.py:269-282) and
+ * ap_out [n_ranges][num_classes] = area under the precision envelope (vid_eval.py:287-343, use_07_metric=False; NaN where
+ * n_pos == 0). prec_out / rec_out [n_ranges][n_det] (may be NULL): class c's curve at the offset of its block in order,
+ * in ranking order; rec_out is written for classes with n_pos > 0 only. Same bits on every run. */
+int mega_vid_eval_scan_ap(const signed char* match, const double* ignore, const int* order, const int* det_count,
+                          const long long* n_pos, long long n_det, long long n_gt, int num_classes, int n_ranges,
+                          void* workspace, long long workspace_bytes, double* prec_out, double* rec_out, double* ap_out,
+                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -226,6 +226,15 @@ lib.mega_dff_warp_scale.argtypes = [_vp, _i, _i, _vp, _i, _vp, _ll, _i, _i, _vp,
 lib.mega_dff_warp_scale.restype = _i
 lib.mega_vid_match_host.argtypes = [_vp, _i, _vp, _vp, _i, _f, ctypes.c_double, _vp, _vp]
 lib.mega_vid_match_host.restype = _i
+lib.mega_vid_eval_workspace_bytes.argtypes = [_ll, _ll, _i, _i]
+lib.mega_vid_eval_workspace_bytes.restype = _ll
+lib.mega_vid_eval_match.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _ll, _ll, _i, _i, _vp, _vp, _f, _vp, _ll,
+                                    _vp, _vp, _vp, _vp, _vp, _vp]
+lib.mega_vid_eval_match.restype = _i
+lib.mega_vid_eval_rank.argtypes = [_ll, _ll, _i, _i, _vp, _ll, _vp, _vp]
+lib.mega_vid_eval_rank.restype = _i
+lib.mega_vid_eval_scan_ap.argtypes = [_vp, _vp, _vp, _vp, _vp, _ll, _ll, _i, _i, _vp, _ll, _vp, _vp, _vp, _vp]
+lib.mega_vid_eval_scan_ap.restype = _i
 
 EXPORTS = [
     "mega_last_error", "mega_abi_version", "mega_device_ok", "mega_conv_gemm", "mega_conv_gemm_tf32", "mega_conv_gemm_workspace_bytes", "mega_set_tf32_rounding",
@@ -241,4 +250,5 @@ EXPORTS = [
     "mega_roi_align_backward_nchw", "mega_roi_pool_forward", "mega_roi_pool_backward", "mega_deform_im2col_kq",
     "mega_deform_col2im_fused", "mega_channel_sum_nchw", "mega_deform_psroi_pooling_backward",
     "mega_image_transform_u8", "mega_dff_warp_scale", "mega_vid_match_host", "mega_split16_pack", "mega_split16_unpack", "mega_relation_softmax_split16", "mega_relation_softmax_pe_split16", "mega_roi_align_forward_nhwc_split16",
+    "mega_vid_eval_workspace_bytes", "mega_vid_eval_match", "mega_vid_eval_rank", "mega_vid_eval_scan_ap",
 ]

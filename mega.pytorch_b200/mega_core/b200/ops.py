@@ -953,3 +953,90 @@ def dff_warp_scale(key_feats, flow, scale, out):
           "mega_dff_warp_scale")
     LAUNCHES[0] += 1
     return out
+
+
+# ---------------------------------------------------------------------------------------------- device VID evaluator
+VID_EVAL_MAX_RANGES = 4
+
+
+def vid_eval_pack(pred_boxlists, gt_boxlists, motion_ious=None):
+    """BoxLists -> flat arrays of mega_vid_eval_match, one torch.cat per field, on the BoxLists' device. motion_ious: per
+    image a sequence of motion IoUs for its GT (or None); entries beyond the GT count are dropped and missing ones are
+    NaN (never ignored), as calc_detection_vid_prec_rec does."""
+    assert len(pred_boxlists) == len(gt_boxlists)
+    det_n = torch.tensor([p.bbox.shape[0] for p in pred_boxlists], dtype=torch.int64)
+    gt_n = torch.tensor([g.bbox.shape[0] for g in gt_boxlists], dtype=torch.int64)
+    zero = torch.zeros(1, dtype=torch.int64)
+    packed = {
+        "det_boxes": torch.cat([p.bbox.reshape(-1, 4) for p in pred_boxlists]).float().contiguous(),
+        "det_scores": torch.cat([p.get_field("scores").reshape(-1) for p in pred_boxlists]).float().contiguous(),
+        "det_labels": torch.cat([p.get_field("labels").reshape(-1) for p in pred_boxlists]).int().contiguous(),
+        "det_off": torch.cat([zero, det_n.cumsum(0)]),
+        "gt_boxes": torch.cat([g.bbox.reshape(-1, 4) for g in gt_boxlists]).float().contiguous(),
+        "gt_labels": torch.cat([g.get_field("labels").reshape(-1) for g in gt_boxlists]).int().contiguous(),
+        "gt_off": torch.cat([zero, gt_n.cumsum(0)]),
+        "gt_motion": None,
+    }
+    if motion_ious is not None:
+        parts = []
+        for m, g in zip(motion_ious, gt_n.tolist()):
+            row = torch.full((g,), float("nan"), dtype=torch.float64)
+            if m is not None and len(m) > 0:
+                m = torch.as_tensor(m, dtype=torch.float64).reshape(-1)[:g]
+                row[:m.numel()] = m
+            parts.append(row)
+        packed["gt_motion"] = torch.cat(parts) if parts else torch.zeros(0, dtype=torch.float64)
+    labels = torch.cat([packed["det_labels"], packed["gt_labels"]])
+    if labels.numel() == 0:
+        raise ValueError("vid_eval: no detections and no ground truth")
+    lo, hi = int(labels.min()), int(labels.max())
+    if lo < 0:
+        raise ValueError("vid_eval: negative class label %d" % lo)
+    packed["num_classes"] = hi + 1
+    return packed
+
+
+def vid_eval(packed, ranges, empty_weights, iou_thresh=0.5, want_prec_rec=False, device="cuda"):
+    """Scores packed BoxLists (vid_eval_pack) for up to 4 motion ranges on the GPU, on the current stream, without
+    synchronising. Returns device tensors: ap [R, C] (NaN where a class has no positives), n_pos [R, C], seen [C] (label
+    occurs: its precision curve exists), det_count [C], order [N] (detections by ascending (class, score); class c's
+    block follows those of the classes below it), match / ignore [R, N], and with want_prec_rec prec / rec [R, N] (class c's
+    curve in ranking order at the offset of its block in order; rec is NaN for classes without positives)."""
+    dev = torch.device(device)
+    r = len(ranges)
+    if not 1 <= r <= VID_EVAL_MAX_RANGES or len(empty_weights) != r:
+        raise _lib.MegaError("vid_eval: 1..%d ranges with one empty weight each" % VID_EVAL_MAX_RANGES)
+    t = {k: (v.to(dev, non_blocking=True) if torch.is_tensor(v) else v) for k, v in packed.items()}
+    require_cuda(t["det_boxes"], t["gt_boxes"])
+    n, g, c = t["det_scores"].numel(), t["gt_labels"].numel(), packed["num_classes"]
+    nbytes = lib.mega_vid_eval_workspace_bytes(n, g, c, r)
+    if nbytes < 0:
+        raise _lib.MegaError("vid_eval: %d detections / %d GT / %d classes / %d ranges exceed the evaluator's limits "
+                             "(< 2^31 boxes, <= 512 classes)" % (n, g, c, r))
+    ws = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=dev)
+    out = {
+        "match": torch.empty(r, n, dtype=torch.int8, device=dev),
+        "ignore": torch.empty(r, n, dtype=torch.float64, device=dev),
+        "n_pos": torch.empty(r, c, dtype=torch.int64, device=dev),
+        "seen": torch.empty(c, dtype=torch.int32, device=dev),
+        "det_count": torch.empty(c, dtype=torch.int32, device=dev),
+        "order": torch.empty(n, dtype=torch.int32, device=dev),
+        "ap": torch.empty(r, c, dtype=torch.float64, device=dev),
+        "prec": torch.empty(r, n, dtype=torch.float64, device=dev) if want_prec_rec else None,
+        "rec": torch.full((r, n), float("nan"), dtype=torch.float64, device=dev) if want_prec_rec else None,
+    }
+    rng = (ctypes.c_double * (2 * r))(*[float(x) for lh in ranges for x in lh])
+    empty = (ctypes.c_double * r)(*[float(x) for x in empty_weights])
+    n_img = t["det_off"].numel() - 1
+    s = stream_ptr()
+    check(lib.mega_vid_eval_match(ptr(t["det_boxes"]), ptr(t["det_scores"]), ptr(t["det_labels"]), ptr(t["det_off"]),
+                                  ptr(t["gt_boxes"]), ptr(t["gt_labels"]), ptr(t["gt_motion"]), ptr(t["gt_off"]), n_img,
+                                  n, g, c, r, rng, empty, float(iou_thresh), ptr(ws), ws.numel(), ptr(out["match"]),
+                                  ptr(out["ignore"]), ptr(out["n_pos"]), ptr(out["seen"]), ptr(out["det_count"]), s),
+          "mega_vid_eval_match")
+    check(lib.mega_vid_eval_rank(n, g, c, r, ptr(ws), ws.numel(), ptr(out["order"]), s), "mega_vid_eval_rank")
+    check(lib.mega_vid_eval_scan_ap(ptr(out["match"]), ptr(out["ignore"]), ptr(out["order"]), ptr(out["det_count"]),
+                                    ptr(out["n_pos"]), n, g, c, r, ptr(ws), ws.numel(), ptr(out["prec"]), ptr(out["rec"]),
+                                    ptr(out["ap"]), s), "mega_vid_eval_scan_ap")
+    LAUNCHES[0] += 2 + 3 * ((32 + (c - 1).bit_length() + 7) // 8)      # match, scan / AP, 3 per radix pass
+    return out

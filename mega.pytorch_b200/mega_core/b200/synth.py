@@ -187,3 +187,60 @@ def global_frame_indices(seg_len, size=10, seed=0):
     a seeded torch permutation here -- only determinism matters for synthetic video)."""
     g = torch.Generator().manual_seed(seed)
     return torch.randperm(seg_len, generator=g).tolist()
+
+
+VID_MOTION_VALUES = (0.3, 0.65, 0.7, 0.8, 0.9, 0.95, 1.0)   # the motion IoUs of tests/golden/vid_eval.pt
+
+
+def vid_eval_set(n_images, seed=0, num_classes=30, max_dets=300, max_gt=5, tie_free=False,
+                 motion_values=VID_MOTION_VALUES, width=640, height=360):
+    """Seeded detections + ground truth for the VID evaluator, vectorised so that validation size (176,126 images) is
+    quick to make. Per image 0..max_gt GT boxes (labels 1..num_classes, motion IoU drawn from motion_values) and
+    0..max_dets detections: jittered copies of GT boxes with high scores and random boxes with the low, long-tailed scores
+    a detector emits after its 1e-3 threshold. tie_free: every score distinct (nudged by ulps).
+    -> (preds, gts, motions): numpy arrays per image, (boxes f32 [n,4], labels i64, scores f32) / (boxes, labels) / list"""
+    import numpy as np
+    rng = np.random.default_rng(seed)
+    n_gt = rng.integers(0, max_gt + 1, n_images)
+    n_det = rng.integers(0, max_dets + 1, n_images)
+    G, N = int(n_gt.sum()), int(n_det.sum())
+    wh = rng.uniform(16, 300, (G, 2))
+    xy = rng.uniform(0, 1, (G, 2)) * (np.array([width, height]) - wh)
+    gt_boxes = np.round(np.concatenate([xy, xy + wh], 1)).astype(np.float32)
+    gt_labels = rng.integers(1, num_classes + 1, G)
+    motion = rng.choice(np.asarray(motion_values, dtype=np.float64), G)
+    gt_img = np.repeat(np.arange(n_images), n_gt)
+    det_img = np.repeat(np.arange(n_images), n_det)
+    gt_first = np.concatenate(([0], np.cumsum(n_gt)))
+    # a detection copies one of its image's GT (jittered) with probability 0.3 when the image has any
+    has_gt = n_gt[det_img] > 0
+    copy = has_gt & (rng.uniform(0, 1, N) < 0.3)
+    src = gt_first[det_img] + (rng.uniform(0, 1, N) * np.maximum(n_gt[det_img], 1)).astype(np.int64)
+    src = np.where(copy, src, 0)
+    wh_d = rng.uniform(8, 300, (N, 2))
+    xy_d = rng.uniform(0, 1, (N, 2)) * (np.array([width, height]) - wh_d)
+    rand_boxes = np.concatenate([xy_d, xy_d + wh_d], 1)
+    g = gt_boxes[src].astype(np.float64) if G else np.zeros((N, 4))
+    jit = rng.normal(0, 0.06, (N, 4)) * (g[:, 2:] - g[:, :2] + 1)[:, [0, 1, 0, 1]]
+    boxes = np.where(copy[:, None], g + jit, rand_boxes)
+    boxes[:, 2:] = np.maximum(boxes[:, 2:], boxes[:, :2])
+    det_boxes = np.clip(boxes, 0, [width - 1, height - 1, width - 1, height - 1]).astype(np.float32)
+    det_labels = np.where(copy & (rng.uniform(0, 1, N) < 0.85), gt_labels[src] if G else 0,
+                          rng.integers(1, num_classes + 1, N))
+    scores = np.where(copy, rng.beta(4.0, 1.5, N), rng.beta(0.4, 6.0, N) * 0.999 + 1e-3).astype(np.float32)
+    if tie_free and N:
+        order = np.argsort(scores, kind="stable")
+        bits = scores[order].view(np.int32).astype(np.int64)
+        ramp = np.arange(N, dtype=np.int64)
+        bits = np.maximum.accumulate(bits - ramp) + ramp
+        scores = np.empty(N, dtype=np.float32)
+        scores[order] = bits.astype(np.int32).view(np.float32)
+    det_first = np.concatenate(([0], np.cumsum(n_det)))
+    preds, gts, motions = [], [], []
+    for i in range(n_images):
+        a, b = det_first[i], det_first[i + 1]
+        c, d = gt_first[i], gt_first[i + 1]
+        preds.append((det_boxes[a:b], det_labels[a:b], scores[a:b]))
+        gts.append((gt_boxes[c:d], gt_labels[c:d]))
+        motions.append(motion[c:d].tolist())
+    return preds, gts, motions
